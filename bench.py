@@ -8,6 +8,7 @@ roughness MLPs, GGX BRDF and the 512-light rendering equation (Stage B) -> sRGB.
 Synthetic data, random-init networks of the reference architecture.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 N > 1 runs under torchrun (one rank per GPU): every rank renders its own full view
 (weak scaling, north star "rays shard naturally"), and one NCCL all-gather per
@@ -50,7 +51,31 @@ def parse():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-secondary', action='store_true',
                     help='skip the bounded secondary measurements (other BASELINE configs)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the arrays the last timed step returned as DIR/<name>.npy (float32)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(pred, out_dir):
+    """Writes every array of one ViewRenderer.render result as <out_dir>/<name>.npy (float32), so
+    that two builds can be compared output for output.  Above DUMP_MAX_BYTES in all, the same
+    seeded sample of rays is kept from every array."""
+    arrs = {k: v.detach().float().cpu().numpy() for k, v in pred.items()
+            if isinstance(v, torch.Tensor)}
+    total = sum(a.nbytes for a in arrs.values())
+    if total > DUMP_MAX_BYTES:
+        n = next(iter(arrs.values())).shape[0]
+        keep = np.sort(np.random.default_rng(0).choice(n, n * DUMP_MAX_BYTES // total, replace=False))
+        arrs = {k: a[keep] for k, a in arrs.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(out_dir, k + '.npy'), np.ascontiguousarray(a))
 
 
 def peaks():
@@ -564,10 +589,14 @@ def main():
             pending[0].wait()
             pending[0] = None
 
+    last_pred = [None]
+
     def step_device():
         pred = vr.render(c2w, synth.CAM_ANGLE_X, args.imh, args.imw)
         if world > 1:
             gather(pred['rgb'])
+        if args.dump_outputs:
+            last_pred[0] = pred
         return pred
 
     def step_e2e():
@@ -610,6 +639,9 @@ def main():
     else:
         ms, launches = timed(step_device, args.steps, max(3, args.warmup))
         clocks = None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last_pred[0], args.dump_outputs)
+    last_pred[0] = None
     ms_step = ms / args.steps
     value = world * n_rays / (ms_step * 1e-3)
     ms_e2e, _ = timed(step_e2e, args.steps, 1)

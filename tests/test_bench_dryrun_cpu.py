@@ -70,6 +70,43 @@ def test_bench_single_rank_line(monkeypatch, capsys):
     assert d['value'] == pytest.approx(64 / (d['ms_per_step'] * 1e-3))
 
 
+def test_bench_dump_outputs_repeatable(monkeypatch, capsys, tmp_path):
+    """--dump-outputs writes the last timed step's render result as float32 .npy files, and two
+    runs with the same arguments write the same arrays."""
+    import numpy as np
+    _patch(monkeypatch)
+    import bench
+    dumps = []
+    for run in ('a', 'b'):
+        monkeypatch.setattr(sys, 'argv', list(ARGV) + ['--dump-outputs', str(tmp_path / run)])
+        bench.main()
+        dumps.append({f[:-4]: np.load(str(tmp_path / run / f))
+                      for f in sorted(os.listdir(str(tmp_path / run)))})
+    capsys.readouterr()
+    assert {'rgb', 'alpha', 'xyz', 'normal', 'albedo', 'brdf'} <= set(dumps[0])
+    for k, a in dumps[0].items():
+        assert a.dtype == np.float32 and a.shape[0] == 64, k
+        assert np.array_equal(a, dumps[1][k]), k
+    assert dumps[0]['alpha'].max() > 0                   # the view has foreground rays
+
+
+def test_dump_outputs_samples_rays_above_the_cap(monkeypatch, tmp_path):
+    import numpy as np
+    if ROOT not in sys.path:
+        sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, 'DUMP_MAX_BYTES', 1000)
+    pred = {'rgb': torch.arange(300.).reshape(100, 3), 'alpha': torch.arange(100.)[:, None],
+            'note': 'not an array'}
+    for run in ('a', 'b'):
+        bench.dump_outputs(pred, str(tmp_path / run))
+    assert sorted(os.listdir(str(tmp_path / 'a'))) == ['alpha.npy', 'rgb.npy']
+    rgb, alpha = np.load(str(tmp_path / 'a' / 'rgb.npy')), np.load(str(tmp_path / 'a' / 'alpha.npy'))
+    assert rgb.nbytes + alpha.nbytes <= 1000 and rgb.shape[0] == alpha.shape[0] > 0
+    assert np.array_equal(rgb[:, 0], 3 * alpha[:, 0])    # the same rays from every array
+    assert np.array_equal(rgb, np.load(str(tmp_path / 'b' / 'rgb.npy')))
+
+
 def _worker(rank, port, q):
     torch.set_num_threads(1)
     os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), RANK=str(rank),

@@ -1,9 +1,9 @@
 """Host-side data formats either side of the hot path (SURVEY.md 8f): dataset classes
 (nerfactor/datasets/{base,nerf,nerf_shape}.py), light-probe loading (nerfactor.py:85-92,
-169-179), image helpers.  Where the reference's own NumPy code is importable
-(/root/reference, build container only) the mirrors are compared with it directly."""
+169-179), image helpers.  The mirrors of the reference's own loaders, writers and image helpers
+are compared with what that code returned on the same inputs (tests/golden/ref_host_code.npz,
+written by tests/golden/make_golden_host.py)."""
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -13,8 +13,11 @@ from nerfactor_b200.datasets import get_dataset_class
 from nerfactor_b200.util import img as imgutil, light as lightutil, io as ioutil, \
     config as configutil
 
-REF = '/root/reference'
 HERE = os.path.dirname(os.path.abspath(__file__))
+
+
+def _golden():
+    return np.load(os.path.join(HERE, 'golden', 'ref_host_code.npz'))
 
 
 def _cfg(root, nerf_root=None, **kw):
@@ -155,28 +158,18 @@ def test_image_helpers_roundtrip(tmp_path):
     assert configutil.get_config_ini('/o/run/checkpoints/ckpt-3') == '/o/run.ini'
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree only in the build container')
 def test_against_importable_reference_helpers(tmp_path):
-    sys.path.insert(0, REF)
-    sys.path.insert(0, os.path.join(HERE, 'golden'))
-    try:
-        import refpin
-        refpin.pin()
-        from third_party.xiuminglib import xiuminglib as xm
-    finally:
-        sys.path.remove(REF)
-        sys.path.remove(os.path.join(HERE, 'golden'))
+    g = _golden()
     rng = np.random.default_rng(3)
     a = rng.random((20, 30, 3))
     u8 = (a * 255).astype(np.uint8)
-    assert np.array_equal(imgutil.normalize_uint(u8), xm.img.normalize_uint(u8))
-    assert np.array_equal(imgutil.denormalize_float(a), xm.img.denormalize_float(a))
+    assert np.array_equal(imgutil.normalize_uint(u8), g['helpers/normalize_uint'])
+    assert np.array_equal(imgutil.denormalize_float(a), g['helpers/denormalize_float'])
     hdr = (rng.random((8, 16, 3)) * 30).astype(np.float32)
-    assert np.array_equal(imgutil.tonemap(hdr, gamma=4), xm.img.tonemap(hdr, gamma=4))
-    assert np.array_equal(imgutil.resize_cv2(a, new_h=10), xm.img.resize(a, new_h=10))
-    assert np.array_equal(imgutil.alpha_blend(a, a[:, :, 0]), xm.img.alpha_blend(a, a[:, :, 0]))
-    assert abs(imgutil.PSNR('uint8')(u8, u8[::-1].copy()) - xm.metric.PSNR('uint8')(
-        u8, u8[::-1].copy())) < 1e-12
+    assert np.array_equal(imgutil.tonemap(hdr, gamma=4), g['helpers/tonemap'])
+    assert np.array_equal(imgutil.resize_cv2(a, new_h=10), g['helpers/resize'])
+    assert np.array_equal(imgutil.alpha_blend(a, a[:, :, 0]), g['helpers/alpha_blend'])
+    assert abs(imgutil.PSNR('uint8')(u8, u8[::-1].copy()) - float(g['helpers/psnr'])) < 1e-12
     lightutil.write_hdr(hdr, str(tmp_path / 'p.hdr'))
     # xm.io.hdr.read itself calls np.fromstring (removed in NumPy 2); same two cv2 calls by hand
     import cv2
@@ -185,112 +178,82 @@ def test_against_importable_reference_helpers(tmp_path):
     assert np.array_equal(lightutil.read_hdr(str(tmp_path / 'p.hdr')), want)
     open(str(tmp_path / 'b.txt'), 'w').close()
     open(str(tmp_path / 'a.txt'), 'w').close()
-    assert ioutil.sortglob(str(tmp_path), '*', ext='txt') == xm.os.sortglob(
-        str(tmp_path), '*', ext='txt')
+    assert [os.path.relpath(p, str(tmp_path)) for p in ioutil.sortglob(
+        str(tmp_path), '*', ext='txt')] == list(g['helpers/sortglob'])
 
 
-# ---- the reference's own loaders / writers, imported through the TensorFlow shim ------------
-def _reference_via_shim():
-    """sys.path set-up for importing /root/reference modules that `import tensorflow` at the
-    top (their loaders / writers are NumPy underneath)."""
-    import warnings
-    warnings.filterwarnings('ignore')
-    paths = [os.path.join(HERE, 'golden', 'tfshim'), REF, os.path.join(REF, 'nerfactor'),
-             os.path.join(HERE, 'golden')]
-    for p in reversed(paths):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    import refpin
-    refpin.pin()          # the reference's namespace packages, not the repo-root drop-in stubs
-    import tensorflow as tf
-    assert tf.__version__.endswith('shim')
-    return paths
+# ---- the reference's own loaders / writers, run on the same inputs by make_golden_host.py ------
+def _rel(files, base):
+    return [os.path.relpath(f, str(base)) for f in files]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree only in the build container')
+def _check_loads(ds, g, pre):
+    """Every view `ds` serves loads to what the reference's loader returned for it."""
+    for i, path in enumerate(ds.files):
+        m = ds._load_data(path)
+        assert m[0] == g[pre + '%d/id' % i].item() and len(m) - 1 == int(g[pre + '%d/n' % i])
+        for j, b in enumerate(m[1:]):
+            a = g[pre + '%d/%d' % (i, j)]
+            assert a.shape == np.shape(b) and np.array_equal(np.asarray(a, np.float32), b), (pre, j)
+
+
 def test_dataset_loaders_equal_reference_loaders(tmp_path):
     """nerfactor/datasets/{nerf,nerf_shape}.py `_glob` + `_load_data` (the reference's files,
     unmodified) vs the loaders here, on a synthetic scene in the reference's layout, incl. the
     resize-on-load path (imh != stored height)."""
-    paths = _reference_via_shim()
-    try:
-        from nerfactor.datasets.nerf import Dataset as RefNerf
-        from nerfactor.datasets.nerf_shape import Dataset as RefShape
-        root, nroot = tmp_path / 'scene', tmp_path / 'surf'
-        synth.write_scene(str(root), imh=16, imw=16, n_train=2, n_val=1, n_test=1,
-                          nerf_root=str(nroot), n_lights=8)
-        for imh in (16, 8):
-            cfg = _cfg(root, nroot, use_nerf_alpha=False, no_batch=True)
-            cfg.set('DEFAULT', 'imh', str(imh))
-            for mode in ('train', 'vali', 'test'):
-                ref = RefShape.__new__(RefShape)            # skip tf.data-related __init__ parts
-                ref.config, ref.mode, ref.debug = cfg, mode, False
-                ref.meta2buf, ref.meta2img, ref.sps = {}, {}, 1
-                ref.files = ref._glob()
-                mine = get_dataset_class('nerf_shape')(cfg, mode)
-                assert mine.files == ref.files
-                for path in ref.files:
-                    r, m = ref._load_data(path), mine._load_data(path)
-                    assert r[0] == m[0]
-                    for a, b in zip(r[1:], m[1:]):
-                        assert a.shape == b.shape and np.array_equal(
-                            np.asarray(a, np.float32), b), (mode, imh)
-            # ray generation incl. the NDC branch and 2 x 2 sub-pixel samples (nerf.py:172-214)
-            for ndc in ('False', 'True'):
-                cfg.set('DEFAULT', 'ndc', ndc)
-                for sps in (1, 2):
-                    rr, mm = RefNerf.__new__(RefNerf), get_dataset_class('nerf').__new__(
-                        get_dataset_class('nerf'))
-                    rr.config = mm.config = cfg
-                    rr.sps = mm.sps = sps
-                    c2w = synth.look_at_c2w(3.0, 40.0, 25.0)
-                    for a, b in zip(rr._gen_rays(c2w, 0.7, 6, 9), mm._gen_rays(c2w, 0.7, 6, 9)):
-                        assert a.shape == b.shape and np.allclose(a, b, rtol=1e-13, atol=1e-13)
-            cfg.set('DEFAULT', 'ndc', 'False')
-            refn = RefNerf.__new__(RefNerf)
-            refn.config, refn.mode, refn.debug, refn.meta2img, refn.sps = cfg, 'train', False, {}, 1
-            refn.files = refn._glob()
-            minen = get_dataset_class('nerf')(cfg, 'train')
-            assert minen.files == refn.files
-            for path in refn.files:
-                r, m = refn._load_data(path), minen._load_data(path)
-                assert r[0] == m[0] and all(np.array_equal(a, b) for a, b in zip(r[1:], m[1:]))
-    finally:
-        for p in paths:
-            sys.path.remove(p)
+    g = _golden()
+    root, nroot = tmp_path / 'scene', tmp_path / 'surf'
+    synth.write_scene(str(root), imh=16, imw=16, n_train=2, n_val=1, n_test=1,
+                      nerf_root=str(nroot), n_lights=8)
+    for imh in (16, 8):
+        cfg = _cfg(root, nroot, use_nerf_alpha=False, no_batch=True)
+        cfg.set('DEFAULT', 'imh', str(imh))
+        for mode in ('train', 'vali', 'test'):
+            pre = 'loaders/shape/%d/%s/' % (imh, mode)
+            mine = get_dataset_class('nerf_shape')(cfg, mode)
+            assert _rel(mine.files, tmp_path) == list(g[pre + 'files'])
+            _check_loads(mine, g, pre)
+        # ray generation incl. the NDC branch and 2 x 2 sub-pixel samples (nerf.py:172-214)
+        for ndc in ('False', 'True'):
+            cfg.set('DEFAULT', 'ndc', ndc)
+            for sps in (1, 2):
+                mm = get_dataset_class('nerf').__new__(get_dataset_class('nerf'))
+                mm.config, mm.sps = cfg, sps
+                c2w = synth.look_at_c2w(3.0, 40.0, 25.0)
+                got = mm._gen_rays(c2w, 0.7, 6, 9)
+                assert len(got) == 2
+                for k, b in enumerate(got):
+                    a = g['loaders/rays/%d/%s/%d/%d' % (imh, ndc, sps, k)]
+                    assert a.shape == b.shape and np.allclose(a, b, rtol=1e-13, atol=1e-13)
+        cfg.set('DEFAULT', 'ndc', 'False')
+        minen = get_dataset_class('nerf')(cfg, 'train')
+        assert _rel(minen.files, tmp_path) == list(g['loaders/nerf/%d/files' % imh])
+        for i, path in enumerate(minen.files):
+            m = minen._load_data(path)
+            assert m[0] == g['loaders/nerf/%d/%d/id' % (imh, i)].item()
+            assert len(m) - 1 == int(g['loaders/nerf/%d/%d/n' % (imh, i)])
+            assert all(np.array_equal(g['loaders/nerf/%d/%d/%d' % (imh, i, j)], b)
+                       for j, b in enumerate(m[1:]))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree only in the build container')
 def test_geometry_buffer_writers_equal_reference_writers(tmp_path):
     """nerfactor/util/geom.py write_alpha / write_xyz / write_normal (and the raw + averaged part
     of write_lvis) vs util/geom_io.py: same .npy bytes, same PNG pixels."""
-    paths = _reference_via_shim()
-    try:
-        from nerfactor.util import geom as refgeom
-        from nerfactor_b200.util import geom_io
-        rng = np.random.default_rng(0)
-        alpha = rng.random((9, 7)).astype(np.float32)
-        xyz = (rng.standard_normal((9, 7, 3)) * alpha[..., None]).astype(np.float32)
-        nrm = rng.standard_normal((9, 7, 3)).astype(np.float32)
-        nrm /= np.linalg.norm(nrm, axis=2, keepdims=True)
-        lvis = rng.random((9, 7, 8)).astype(np.float32)
-        rd, md = str(tmp_path / 'ref'), str(tmp_path / 'mine')
-        os.makedirs(rd)
-        refgeom.write_alpha(alpha, rd)
-        refgeom.write_xyz(xyz, rd)
-        refgeom.write_normal(nrm, rd)
-        np.save(os.path.join(rd, 'lvis.npy'), lvis)             # geom.py:30-32
-        from third_party.xiuminglib import xiuminglib as xm
-        xm.io.img.write_arr(np.mean(lvis, axis=2), os.path.join(rd, 'lvis.png'))   # geom.py:34-36
-        geom_io.write_view_buffers({'alpha': alpha, 'xyz': xyz, 'normal': nrm, 'lvis': lvis}, md)
-        for f in ('xyz.npy', 'normal.npy', 'lvis.npy'):
-            assert open(os.path.join(rd, f), 'rb').read() == open(os.path.join(md, f), 'rb').read()
-        for f in ('alpha.png', 'xyz.png', 'normal.png', 'lvis.png'):
-            a, b = imgutil.read(os.path.join(rd, f)), imgutil.read(os.path.join(md, f))
-            assert a.shape == b.shape and np.array_equal(a, b), f
-    finally:
-        for p in paths:
-            sys.path.remove(p)
+    from nerfactor_b200.util import geom_io
+    g = _golden()
+    rng = np.random.default_rng(0)
+    alpha = rng.random((9, 7)).astype(np.float32)
+    xyz = (rng.standard_normal((9, 7, 3)) * alpha[..., None]).astype(np.float32)
+    nrm = rng.standard_normal((9, 7, 3)).astype(np.float32)
+    nrm /= np.linalg.norm(nrm, axis=2, keepdims=True)
+    lvis = rng.random((9, 7, 8)).astype(np.float32)
+    md = str(tmp_path / 'mine')
+    geom_io.write_view_buffers({'alpha': alpha, 'xyz': xyz, 'normal': nrm, 'lvis': lvis}, md)
+    for f in ('xyz.npy', 'normal.npy', 'lvis.npy'):
+        assert open(os.path.join(md, f), 'rb').read() == g['writers/' + f].tobytes(), f
+    for f in ('alpha.png', 'xyz.png', 'normal.png', 'lvis.png'):
+        a, b = g['writers/' + f], imgutil.read(os.path.join(md, f))
+        assert a.shape == b.shape and np.array_equal(a, b), f
 
 
 def _write_mvs_scene(root, imh=8):
@@ -327,26 +290,12 @@ def test_mvs_shape_dataset(tmp_path):
     assert np.allclose(np.linalg.norm(rayo.numpy(), axis=1), 4., atol=1e-5)   # the camera location
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree only in the build container')
 def test_mvs_shape_loader_equals_reference_loader(tmp_path):
-    paths = _reference_via_shim()
-    try:
-        from nerfactor.datasets.mvs_shape import Dataset as RefMvs
-        root = tmp_path / 'mvs'
-        _write_mvs_scene(root)
-        cfg = _cfg(tmp_path / 'unused', None, mvs_root=str(root), use_nerf_alpha=False)
-        for mode in ('train', 'vali', 'test'):
-            ref = RefMvs.__new__(RefMvs)
-            ref.config, ref.mode, ref.debug, ref.meta2buf, ref.meta2img, ref.sps = \
-                cfg, mode, False, {}, {}, 1
-            ref.files = ref._glob()
-            mine = get_dataset_class('mvs_shape')(cfg, mode)
-            assert mine.files == ref.files and ref.files
-            for path in ref.files:
-                r, m = ref._load_data(path), mine._load_data(path)
-                assert r[0] == m[0]
-                for a, b in zip(r[1:], m[1:]):
-                    assert a.shape == b.shape and np.array_equal(np.asarray(a, np.float32), b)
-    finally:
-        for p in paths:
-            sys.path.remove(p)
+    g = _golden()
+    root = tmp_path / 'mvs'
+    _write_mvs_scene(root)
+    cfg = _cfg(tmp_path / 'unused', None, mvs_root=str(root), use_nerf_alpha=False)
+    for mode in ('train', 'vali', 'test'):
+        mine = get_dataset_class('mvs_shape')(cfg, mode)
+        assert _rel(mine.files, tmp_path) == list(g['mvs/%s/files' % mode]) and mine.files
+        _check_loads(mine, g, 'mvs/%s/' % mode)

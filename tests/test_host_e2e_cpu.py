@@ -148,24 +148,30 @@ def test_trainer_gradients_equal_reference_tape(monkeypatch, kind):
 
 import os as _os
 
-_REF_CFG = '/root/reference/nerfactor/config'
+_GOLDEN = _os.path.join(_os.path.dirname(_os.path.abspath(__file__)), 'golden', 'ref_host_code.npz')
 
 
-@pytest.mark.skipif(not _os.path.isdir(_REF_CFG), reason='reference tree only in the build container')
 @pytest.mark.parametrize('ini', ['nerfactor.ini', 'nerfactor_microfacet.ini', 'nerfactor_mvs.ini',
                                  'nerfactor_no_geom_opt.ini', 'nerfactor_no_geom_pretrain.ini',
                                  'nerfactor_no_smooth.ini', 'shape.ini', 'shape_mvs.ini',
                                  'nerf.ini', 'brdf.ini'])
 def test_every_shipped_reference_config_drives_the_models(monkeypatch, tmp_path, ini):
-    """The reference's own .ini files (read as they are, site paths replaced): model construction,
-    a forward pass and the loss on the CPU test double -- every key the models read is present or
-    has the reference's fallback."""
+    """The reference's own .ini files (their keys and values as stored by
+    tests/golden/make_golden_host.py, written back to an .ini and read as such, site paths
+    replaced): model construction, a forward pass and the loss on the CPU test double -- every key
+    the models read is present or has the reference's fallback."""
+    import json
+    from configparser import ConfigParser
     import numpy as _np
     from nerfactor_b200 import models
     from nerfactor_b200.brdf.renderer import gen_light_xyz
     from nerfactor_b200.util import io as ioutil
     ctx = cpu_backend.install(monkeypatch)
-    cfg = ioutil.read_config(_os.path.join(_REF_CFG, ini))
+    stored = ConfigParser()
+    stored.read_dict(json.loads(str(np.load(_GOLDEN)['configs/' + ini])))
+    with open(str(tmp_path / ini), 'w') as h:
+        stored.write(h)
+    cfg = ioutil.read_config(str(tmp_path / ini))
     lh = 2
     for k in ('data_root', 'data_nerf_root', 'outroot', 'test_envmap_dir'):
         if cfg.has_option('DEFAULT', k):

@@ -2,7 +2,6 @@
 of the models' `vis_batch` / `compile_batch_vis` (SURVEY.md 8f.4): everything that does not need
 the GPU.  The end-to-end run of the three scripts on a B200 is tests/test_zz_gpu_scripts.py."""
 import os
-import sys
 from collections import OrderedDict
 
 import numpy as np
@@ -14,7 +13,7 @@ from nerfactor_b200 import trainvali, geometry_from_nerf as gfn
 from nerfactor_b200.models._visualize import NeRFactorVis, ShapeVis, NerfVis
 from nerfactor_b200.util import img as imgutil, io as ioutil
 
-REF = '/root/reference'
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'ref_host_code.npz')
 
 
 # ------------------------------------------------------------------------------ test.py
@@ -36,21 +35,14 @@ def test_albedo_overrides():
         nftest.get_albedo_override(xyz, 'plaid')
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree only in the build container')
 def test_turbo_fit_against_reference_table():
-    sys.path.insert(0, REF)
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
-    import refpin
-    refpin.pin()
-    try:
-        from third_party.turbo_colormap import turbo_colormap_data, interpolate_or_clip
-    finally:
-        sys.path.remove(REF)
+    """nftest.turbo vs the reference's turbo table and its interpolate_or_clip
+    (third_party/turbo_colormap.py), values stored by tests/golden/make_golden_host.py."""
+    g = np.load(GOLDEN)
     xs = np.linspace(0, 1, 501)
-    want = np.array([interpolate_or_clip(turbo_colormap_data, float(x)) for x in xs])
-    assert np.abs(nftest.turbo(xs) - want).max() < 0.011
-    assert interpolate_or_clip(turbo_colormap_data, -0.1) == [0.0, 0.0, 0.0]
-    assert interpolate_or_clip(turbo_colormap_data, 1.1) == [1.0, 1.0, 1.0]
+    assert np.abs(nftest.turbo(xs) - g['turbo/table']).max() < 0.011
+    assert list(g['turbo/below']) == [0.0, 0.0, 0.0]
+    assert list(g['turbo/above']) == [1.0, 1.0, 1.0]
 
 
 def test_compute_rgb_scales(tmp_path):
@@ -231,147 +223,74 @@ def test_nerf_vis_batch(tmp_path):
     assert m.compile_batch_vis([vdir], str(tmp_path / 'e' / 'vid'), 'test').endswith('.mp4')
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree only in the build container')
 def test_vis_batch_equals_reference_vis_batch(tmp_path, monkeypatch):
     """The reference's NeRFactor `vis_batch` (nerfactor.py:562-739, its own file, run through the
-    TensorFlow shim on the reference model's own outputs) vs `vis_batch` here on the same
-    `to_vis`: same files, same pixels (text-free images), incl. OLAT / probe renders composited
-    on the average light and the per-light visibility maps."""
-    import warnings
-    warnings.filterwarnings('ignore')
-    here = os.path.dirname(os.path.abspath(__file__))
-    paths = [os.path.join(here, 'golden', 'tfshim'), REF, os.path.join(REF, 'nerfactor'),
-             os.path.join(here, 'golden')]
-    for p in reversed(paths):
-        sys.path.insert(0, p)
-    try:
-        sys.path.insert(0, os.path.join(here, 'golden'))
-        import refpin
-        refpin.pin()      # the reference's namespace packages, not the repo-root drop-in stubs
-        import tensorflow as tf
-        assert tf.__version__.endswith('shim')
-        import make_golden_tfshim as gen
-        import torch
-        from nerfactor_b200 import synth
-        lh, h, w = 2, 6, 5
-        model, cfg, params = gen.build_stage_b('microfacet', lh, str(tmp_path / 'cfg'), 7)
-        L = 2 * lh * lh
-        batch_np = list(synth.make_stage_b_batch(11, h * w, L))
-        batch_np[1] = np.tile(np.array([[h, w]], np.int32), (h * w, 1))
-
-        class _Id:                                   # an eager string tensor: x[0].numpy() -> bytes
-            def __getitem__(self, i):
-                return self
-
-            def numpy(self):
-                return b'test_007'
-        batch = tuple(_Id() if i == 0 else gen.t32(x) if i > 1 else torch.as_tensor(x)
-                      for i, x in enumerate(batch_np))
-        probes = synth.make_probes(5, 2, (lh, 2 * lh))
-        from collections import OrderedDict
-        model.novel_probes = OrderedDict(('p%d' % i, gen.t32(p)) for i, p in enumerate(probes))
-        from nerfactor.util import light as reflight
-        model.novel_probes_uint = {k: reflight.vis_light(v, h=model.embed_light_h)
-                                   for k, v in model.novel_probes.items()}
-        _, _, _, to_vis = model.call(batch, mode='test', relight_olat=True, relight_probes=True)
-        mine_in = {k: (v.detach().numpy().copy() if isinstance(v, torch.Tensor) else v)
-                   for k, v in to_vis.items()}
-        mine_in['id'], mine_in['hw'] = 'test_007', (h, w)
-        rdir, mdir = str(tmp_path / 'ref'), str(tmp_path / 'mine')
-        model.vis_batch(to_vis, rdir, mode='test', olat_vis=True)
-        # ---- the model here (host code only: vis_batch never touches the kernels)
-        import cpu_backend
-        ctx = cpu_backend.install(monkeypatch)
-        from nerfactor_b200.models.nerfactor_microfacet import Model
-        m = Model(nfconfig.default_config('nerfactor_microfacet', light_h=lh), params=params,
-                  ctx=ctx, precision='fp32')
-        for i, p in enumerate(probes):
-            m.novel_probes['p%d' % i] = torch.as_tensor(p)
-        m.vis_batch(mine_in, mdir, mode='test', olat_vis=True)
-        rf, mf = sorted(os.listdir(rdir)), sorted(os.listdir(mdir))
-        assert rf == mf and len(rf) > 20
-        assert ioutil.read_json(os.path.join(rdir, 'metadata.json')) == ioutil.read_json(
-            os.path.join(mdir, 'metadata.json'))
-        for f in rf:
-            if f.endswith('.png'):
-                a = imgutil.read(os.path.join(rdir, f)).astype(int)
-                b = imgutil.read(os.path.join(mdir, f)).astype(int)
-                assert a.shape == b.shape and np.abs(a - b).max() <= 1, f
-    finally:
-        for p in paths:
-            sys.path.remove(p)
+    TensorFlow shim on the reference model's own outputs by tests/golden/make_golden_host.py) vs
+    `vis_batch` here on the same `to_vis`: same files, same pixels (text-free images), incl. OLAT /
+    probe renders composited on the average light and the per-light visibility maps."""
+    import json
+    import torch
+    import cpu_backend
+    from nerfactor_b200 import synth
+    from nerfactor_b200.models.nerfactor_microfacet import Model
+    g = np.load(GOLDEN)
+    lh, h, w = 2, 6, 5
+    params = synth.make_stage_b_params(7, 'microfacet', light_hw=(lh, 2 * lh))
+    probes = synth.make_probes(5, 2, (lh, 2 * lh))
+    mine_in = {k[len('vis/in/'):]: g[k].copy() for k in g.files if k.startswith('vis/in/')}
+    mine_in['id'], mine_in['hw'] = 'test_007', (h, w)
+    mdir = str(tmp_path / 'mine')
+    # ---- the model here (host code only: vis_batch never touches the kernels)
+    ctx = cpu_backend.install(monkeypatch)
+    m = Model(nfconfig.default_config('nerfactor_microfacet', light_h=lh), params=params,
+              ctx=ctx, precision='fp32')
+    for i, p in enumerate(probes):
+        m.novel_probes['p%d' % i] = torch.as_tensor(p)
+    m.vis_batch(mine_in, mdir, mode='test', olat_vis=True)
+    rf, mf = list(g['vis/files']), sorted(os.listdir(mdir))
+    assert rf == mf and len(rf) > 20
+    assert json.loads(str(g['vis/metadata'])) == ioutil.read_json(os.path.join(mdir, 'metadata.json'))
+    for f in rf:
+        if f.endswith('.png'):
+            a = g['vis/png/' + f].astype(int)
+            b = imgutil.read(os.path.join(mdir, f)).astype(int)
+            assert a.shape == b.shape and np.abs(a - b).max() <= 1, f
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree only in the build container')
 def test_stage_a_files_equal_reference_process_view(tmp_path, monkeypatch):
     """geometry_from_nerf.process_view of the reference (its own file through the shim: march,
     occupancy threshold, alpha / xyz / normal maps, hit mask, light visibility, alpha masking,
-    file writers) vs `process_view` + `write_view_buffers` here on the CPU test double: the four
-    buffers a Stage-B dataset reads."""
-    import warnings
-    warnings.filterwarnings('ignore')
-    here = os.path.dirname(os.path.abspath(__file__))
-    paths = [os.path.join(here, 'golden', 'tfshim'), REF, os.path.join(REF, 'nerfactor'),
-             os.path.join(here, 'golden')]
-    for p in reversed(paths):
-        sys.path.insert(0, p)
-    try:
-        import tensorflow as tf
-        import torch
-        import make_golden_tfshim as gen
-        from nerfactor import geometry_from_nerf as refgfn
-        from nerfactor.models.nerf import Model as RefNerf
-        from third_party.xiuminglib import xiuminglib as xm
-        from nerfactor_b200 import synth
-        from oracle import stage_a
-        monkeypatch.setattr(xm.vis.video, 'make_video', lambda *a, **k: None)   # lvis.mp4: vis only
-        lh, h, w = 2, 5, 6
-        rdir, mdir = str(tmp_path / 'ref'), str(tmp_path / 'mine')
-        if not refgfn.FLAGS.is_parsed():
-            refgfn.FLAGS(['t'])
-        refgfn.FLAGS.light_h, refgfn.FLAGS.out_root = lh, rdir
-        refgfn.FLAGS.occu_thres, refgfn.FLAGS.spp = 0.9, 1
-        cfg = gen.read_ini('nerf.ini', n_samples_coarse=-48, n_samples_fine=8, data_root='/tmp',
-                           outroot='/tmp')
-        ref_model = RefNerf(cfg)
-        params = synth.make_nerf_params(3)
-        gen.set_weights(ref_model.net, params)
-        rayo, rayd = stage_a.gen_rays(synth.look_at_c2w(), synth.CAM_ANGLE_X, h, w)
-        rayo, rayd = rayo.reshape(-1, 3), rayd.reshape(-1, 3)
-
-        class _Id:
-            def __getitem__(self, i):
-                return self
-
-            def numpy(self):
-                return b'train_003'
-        batch = (_Id(), torch.tensor([[h, w]] * (h * w), dtype=torch.int32), gen.t32(rayo),
-                 gen.t32(rayd), None)
-        refgfn.process_view(cfg, ref_model, batch)
-        # ---- here, kernels replaced by the test double
-        import cpu_backend
-        ctx = cpu_backend.install(monkeypatch)
-        from nerfactor_b200 import geometry_from_nerf as gfn
-        from nerfactor_b200.models.nerf import Model
-        from nerfactor_b200.util import geom_io
-        model = Model(nfconfig.default_config('nerf', n_samples_coarse=-48, n_samples_fine=8),
-                      params=params, ctx=ctx, precision='fp32')
-        ro = torch.as_tensor(rayo)
-        rd = torch.as_tensor(rayd)
-        rd = rd * torch.rsqrt(torch.clamp((rd * rd).sum(1, keepdim=True), min=1e-12))
-        buffers = gfn.process_view(model, ro, rd, (h, w), model.config, occu_thres=0.9,
-                                   lvis_far=1., light_h=lh, precision='fp32')
-        geom_io.write_view_buffers(buffers, os.path.join(mdir, 'train_003'))
-        rd_, md_ = os.path.join(rdir, 'train_003'), os.path.join(mdir, 'train_003')
-        assert geom_io.view_done(rd_) and geom_io.view_done(md_)
-        a_r = imgutil.read(os.path.join(rd_, 'alpha.png')).astype(int)
-        a_m = imgutil.read(os.path.join(md_, 'alpha.png')).astype(int)
-        assert a_r.shape == a_m.shape and np.abs(a_r - a_m).max() <= 1
-        assert 0 < (a_r > 0).mean() < 1                   # the threshold removed some pixels
-        for f, tol in (('xyz.npy', 2e-5), ('normal.npy', 2e-4), ('lvis.npy', 5e-5)):
-            r, m_ = np.load(os.path.join(rd_, f)), np.load(os.path.join(md_, f))
-            assert r.shape == m_.shape and r.dtype == m_.dtype == np.float32
-            assert np.abs(r - m_).max() < tol, (f, np.abs(r - m_).max())
-    finally:
-        for p in paths:
-            sys.path.remove(p)
+    file writers; stored by tests/golden/make_golden_host.py) vs `process_view` +
+    `write_view_buffers` here on the CPU test double: the four buffers a Stage-B dataset reads."""
+    import torch
+    import cpu_backend
+    from nerfactor_b200 import synth
+    from nerfactor_b200.models.nerf import Model
+    from nerfactor_b200.util import geom_io
+    from oracle import stage_a
+    g = np.load(GOLDEN)
+    lh, h, w = 2, 5, 6
+    mdir = str(tmp_path / 'mine')
+    params = synth.make_nerf_params(3)
+    rayo, rayd = stage_a.gen_rays(synth.look_at_c2w(), synth.CAM_ANGLE_X, h, w)
+    rayo, rayd = rayo.reshape(-1, 3), rayd.reshape(-1, 3)
+    # ---- here, kernels replaced by the test double
+    ctx = cpu_backend.install(monkeypatch)
+    model = Model(nfconfig.default_config('nerf', n_samples_coarse=-48, n_samples_fine=8),
+                  params=params, ctx=ctx, precision='fp32')
+    ro = torch.as_tensor(rayo)
+    rd = torch.as_tensor(rayd)
+    rd = rd * torch.rsqrt(torch.clamp((rd * rd).sum(1, keepdim=True), min=1e-12))
+    buffers = gfn.process_view(model, ro, rd, (h, w), model.config, occu_thres=0.9,
+                               lvis_far=1., light_h=lh, precision='fp32')
+    md_ = os.path.join(mdir, 'train_003')
+    geom_io.write_view_buffers(buffers, md_)
+    assert geom_io.view_done(md_)
+    a_r = g['process_view/alpha.png'].astype(int)
+    a_m = imgutil.read(os.path.join(md_, 'alpha.png')).astype(int)
+    assert a_r.shape == a_m.shape and np.abs(a_r - a_m).max() <= 1
+    assert 0 < (a_r > 0).mean() < 1                   # the threshold removed some pixels
+    for f, tol in (('xyz.npy', 2e-5), ('normal.npy', 2e-4), ('lvis.npy', 5e-5)):
+        r, m_ = g['process_view/' + f], np.load(os.path.join(md_, f))
+        assert r.shape == m_.shape and r.dtype == m_.dtype == np.float32
+        assert np.abs(r - m_).max() < tol, (f, np.abs(r - m_).max())

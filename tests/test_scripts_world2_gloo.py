@@ -17,8 +17,10 @@ def _worker(rank, world, port, tmp, q):
     for p in (HERE, os.path.dirname(HERE)):
         if p not in sys.path:
             sys.path.insert(0, p)
+    # CUDA_VISIBLE_DEVICES='': the kernels are the CPU test double, so the scripts must not pick
+    # cuda:<LOCAL_RANK> (which does not exist on a one-GPU machine) either
     os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), RANK=str(rank),
-                      WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
+                      WORLD_SIZE=str(world), LOCAL_RANK=str(rank), CUDA_VISIBLE_DEVICES='')
     import cpu_backend
     mpatch = pytest.MonkeyPatch()
     cpu_backend.install(mpatch)
@@ -88,8 +90,10 @@ def _train_worker(rank, world, port, ini, q):
     for p in (HERE, os.path.dirname(HERE)):
         if p not in sys.path:
             sys.path.insert(0, p)
+    # CUDA_VISIBLE_DEVICES='': the kernels are the CPU test double, so the scripts must not pick
+    # cuda:<LOCAL_RANK> (which does not exist on a one-GPU machine) either
     os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), RANK=str(rank),
-                      WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
+                      WORLD_SIZE=str(world), LOCAL_RANK=str(rank), CUDA_VISIBLE_DEVICES='')
     import cpu_backend
     mpatch = pytest.MonkeyPatch()
     cpu_backend.install(mpatch)
