@@ -166,6 +166,39 @@ typedef struct nf_integrate_args {
 } nf_integrate_args;
 int nf_integrate_fwd(nf_ctx* ctx, const nf_integrate_args* args, void* stream);
 
+/* Backward of nf_integrate_fwd for one env-map: given d_rgb = dE/d rgb, the gradients torch
+ * autograd (or TF's tape) takes through the reference formulas -- Microfacet.__call__
+ * (brdf/microfacet/microfacet.py:30-111) or albedo/pi + spec*scale (nerfactor.py:457-461), then
+ * nerfactor.py:315-342 -- with these conventions: the gates cos > 0, chi_d, chi_g have zero
+ * derivative; divide_no_nan gives 0 value and gradient where its denominator is 0; d|x| = sign(x)
+ * with sign(0) = 0; the clip to [0, 1] passes the gradient on the closed interval; linear2srgb
+ * takes the slope of the selected branch; rough enters through alpha = rough^2.
+ *   d_normal_d is with respect to the RAW normal_d, through both normalisations (nerfactor.py:212
+ *   and microfacet.py:47); d_spec_d (brdf_kind 1) is with respect to spec_d before spec_scale;
+ *   d_light_d [L,3] is summed over the n points.  No gradient is taken with respect to xyz_d,
+ *   cam_d, lxyz_d or lareas_d.
+ * Restrictions: n_envmaps == 1, light_idx_d == NULL, envmap_pixels == n_lights (gather the texels
+ * per light first); anything else is NF_ERR_UNSUPPORTED.  `args->rgb_d` is not read: the linear
+ * sum is recomputed from the inputs, nothing of the forward call needs to be kept.
+ * A NULL output is neither computed nor written (d_lvis_d / d_spec_d are the [n, L] writes);
+ * outputs are overwritten, not accumulated into.  workspace_d: nf_integrate_bwd_workspace_bytes()
+ * bytes, needed only when d_light_d is requested (per-block partial sums of d_light, added in a
+ * fixed order: results are bit-identical from run to run).  No allocation, no synchronisation
+ * (CUDA-graph capturable).  The workspace query is host-only and returns 0 for an unsupported
+ * argument block.                                                                              */
+typedef struct nf_integrate_grads {
+  const float* d_rgb_d;   /* [n,3]  upstream gradient of the tonemapped rgb                       */
+  float* d_lvis_d;        /* [n,L]  or NULL                                                       */
+  float* d_normal_d;      /* [n,3]  w.r.t. the raw normal_d, or NULL                              */
+  float* d_albedo_d;      /* [n,3]  or NULL                                                       */
+  float* d_rough_d;       /* [n]    brdf_kind 0, or NULL                                          */
+  float* d_spec_d;        /* [n,L]  brdf_kind 1 (w.r.t. spec_d before spec_scale), or NULL        */
+  float* d_light_d;       /* [L,3]  summed over the n points, or NULL                             */
+} nf_integrate_grads;
+size_t nf_integrate_bwd_workspace_bytes(const nf_integrate_args* args);
+int nf_integrate_bwd(nf_ctx* ctx, const nf_integrate_args* args, const nf_integrate_grads* grads,
+                     void* workspace_d, size_t workspace_bytes, void* stream);
+
 /* One-light-at-a-time relighting: rgb_olat[n, L, 3] for the L env-maps
  * olat_inten * onehot(l) + ambient (nerfactor/models/nerfactor.py:71-84, 348-354),
  * same argument block (light_d / n_envmaps ignored). */

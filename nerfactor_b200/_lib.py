@@ -33,7 +33,8 @@ EXPORTS = [
     'nf_adam_amsgrad_step', 'nf_microfacet_brdf_fwd', 'nf_selftest_tmem',
     'nf_raymarch_depth_normal_workspace_bytes', 'nf_raymarch_depth_normal_fwd',
     'nf_raymarch_lvis_workspace_bytes', 'nf_raymarch_lvis_fwd',
-    'nf_stageB_fused_workspace_bytes', 'nf_stageB_fused_fwd', 'nf_lvis_dirs_fwd', 'nf_lvis_inputs_fwd']
+    'nf_stageB_fused_workspace_bytes', 'nf_stageB_fused_fwd', 'nf_lvis_dirs_fwd', 'nf_lvis_inputs_fwd',
+    'nf_integrate_bwd_workspace_bytes', 'nf_integrate_bwd']
 
 
 class NfError(RuntimeError):
@@ -63,6 +64,12 @@ class IntegrateArgs(C.Structure):
                 ('albedo_d', C.c_void_p), ('rough_d', C.c_void_p), ('spec_d', C.c_void_p),
                 ('lvis_d', C.c_void_p), ('lxyz_d', C.c_void_p), ('lareas_d', C.c_void_p),
                 ('light_d', C.c_void_p), ('light_idx_d', C.c_void_p), ('rgb_d', C.c_void_p)]
+
+
+class IntegrateGrads(C.Structure):
+    _fields_ = [('d_rgb_d', C.c_void_p), ('d_lvis_d', C.c_void_p), ('d_normal_d', C.c_void_p),
+                ('d_albedo_d', C.c_void_p), ('d_rough_d', C.c_void_p), ('d_spec_d', C.c_void_p),
+                ('d_light_d', C.c_void_p)]
 
 
 class StageBArgs(C.Structure):
@@ -123,6 +130,10 @@ def load_library():
     lib.nf_brdf_learned_fwd.argtypes = [vp, vp, vp, vp, vp, vp, i, vp, i, vp, i, vp]
     lib.nf_integrate_fwd.argtypes = [vp, C.POINTER(IntegrateArgs), vp]
     lib.nf_integrate_olat_fwd.argtypes = [vp, C.POINTER(IntegrateArgs), f, f, vp, vp]
+    lib.nf_integrate_bwd_workspace_bytes.argtypes = [C.POINTER(IntegrateArgs)]
+    lib.nf_integrate_bwd_workspace_bytes.restype = C.c_size_t
+    lib.nf_integrate_bwd.argtypes = [vp, C.POINTER(IntegrateArgs), C.POINTER(IntegrateGrads), vp,
+                                     C.c_size_t, vp]
     lib.nf_microfacet_brdf_fwd.argtypes = [vp, vp, vp, vp, vp, vp, i, i, f, i, f, vp, vp]
     lib.nf_gen_rays.argtypes = [vp, C.POINTER(d), d, i, i, i, vp, vp, vp]
     lib.nf_gen_z.argtypes = [vp, f, f, i, i, i, vp, vp, vp]
@@ -159,7 +170,8 @@ def load_library():
         if name not in ('nf_last_error_string', 'nf_mlp_device_bytes',
                         'nf_dense_bwd_workspace_bytes', 'nf_dense_fwd_workspace_bytes',
                         'nf_raymarch_depth_normal_workspace_bytes',
-                        'nf_raymarch_lvis_workspace_bytes', 'nf_stageB_fused_workspace_bytes'):
+                        'nf_raymarch_lvis_workspace_bytes', 'nf_stageB_fused_workspace_bytes',
+                        'nf_integrate_bwd_workspace_bytes'):
             getattr(lib, name).restype = i
     _lib = lib
     return lib
@@ -370,6 +382,35 @@ def integrate_fwd(ctx, xyz, normal, cam, albedo, lvis, lxyz, lareas, light, roug
                         light_idx, rgb, f0, spec_scale, linear2srgb)
     ctx.launch(ctx.lib.nf_integrate_fwd(ctx.h, C.byref(a), _stream()))
     return rgb
+
+
+def integrate_bwd(ctx, xyz, normal, cam, albedo, lvis, lxyz, lareas, light, d_rgb, rough=None,
+                  spec=None, f0=0.04, spec_scale=1.0, linear2srgb=True, need=()):
+    """Gradients of integrate_fwd with one env-map, light [L, 3] (one texel per light, >= 0), given
+    d_rgb [n, 3].  `need`: names out of 'lvis', 'normal', 'albedo', 'rough' (with rough), 'spec'
+    (with spec), 'light'; only those are computed.  -> {name: gradient} (normal: with respect to
+    the raw normal, spec: before spec_scale, light: summed over the points, rough: shape of rough)."""
+    n, L = xyz.shape[0], lxyz.reshape(-1, 3).shape[0]
+    light = light.reshape(1, L, 3)
+    a = _integrate_args(xyz, normal, cam, albedo, lvis, lxyz, lareas,
+                        None if rough is None else rough.reshape(-1), spec, light, None, None, f0,
+                        spec_scale, linear2srgb)
+    shapes = {'lvis': (n, L), 'normal': (n, 3), 'albedo': (n, 3), 'light': (L, 3),
+              'rough': (n,), 'spec': (n, L)}
+    out = {k: torch.empty(shapes[k], dtype=torch.float32, device=xyz.device) for k in need}
+    g = IntegrateGrads()
+    g.d_rgb_d = _f32(d_rgb)
+    for k, t in out.items():
+        setattr(g, 'd_%s_d' % k, _f32(t))
+    nbytes = ctx.lib.nf_integrate_bwd_workspace_bytes(C.byref(a)) if 'light' in out else 0
+    work = torch.empty((nbytes,), dtype=torch.uint8, device=xyz.device) if nbytes else None
+    if 'light' in out:
+        ctx.launches += 1                    # the ordered sum of the per-block d_light partials
+    ctx.launch(ctx.lib.nf_integrate_bwd(ctx.h, C.byref(a), C.byref(g), _ptr(work), nbytes,
+                                        _stream()))
+    if 'rough' in out:
+        out['rough'] = out['rough'].reshape(rough.shape)
+    return out
 
 
 def integrate_olat_fwd(ctx, xyz, normal, cam, albedo, lvis, lxyz, lareas, olat_inten,

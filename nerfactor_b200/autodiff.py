@@ -3,7 +3,8 @@
 A train step works on `n_rays_per_step` = 1024 rays (nerfactor.ini:93), i.e. 0.5 M
 (ray, light) rows -- three orders of magnitude less than a test-time view.  The Dense
 contractions (>99.9 % of the step's FLOPs) run in this library's CUDA kernels through
-`DenseFn` (nf_dense_fwd / nf_dense_bwd); the O(N L) element-wise rendering math around
+`DenseFn` (nf_dense_fwd / nf_dense_bwd), the rendering equation through `IntegrateFn`
+(nf_integrate_fwd / nf_integrate_bwd); the rest of the O(N L) element-wise math around
 them is expressed in torch ops on the device so torch.autograd provides its adjoint,
 with the reference's custom gradients (nerfactor/util/math.py:24-60) kept as explicit
 autograd Functions.  Forward values equal the fused inference kernels' (same formulas).
@@ -283,3 +284,57 @@ def render(lvis, brdf, surf2l, normal, light_flat, lareas, srgb):
         lareas.reshape(1, -1, 1)
     rgb = torch.clamp(torch.sum(contrib, dim=1), 0., 1.)
     return linear2srgb(rgb) if srgb else rgb
+
+
+class IntegrateFn(torch.autograd.Function):
+    """The rendering equation through nf_integrate_fwd, its adjoint through nf_integrate_bwd (only
+    the gradients autograd asks for; the backward recomputes the sum from the saved inputs)."""
+
+    @staticmethod
+    def forward(ctx, lvis, normal, albedo, brdf_prop, light_flat, xyz, cam, lxyz, lareas, kind,
+                f0, spec_scale, srgb):
+        c = _lib.default_context()
+        ins = [t.contiguous() for t in (lvis, normal, albedo, brdf_prop, light_flat, xyz, cam,
+                                        lxyz.reshape(-1, 3), lareas.reshape(-1))]
+        lvis, normal, albedo, prop, light_flat, xyz, cam, lxyz, lareas = ins
+        rough, spec = (prop, None) if kind == 0 else (None, prop)
+        rgb = _lib.integrate_fwd(c, xyz, normal, cam, albedo, lvis, lxyz, lareas,
+                                 light_flat.reshape(1, -1, 3), rough=rough, spec=spec, f0=f0,
+                                 spec_scale=spec_scale, linear2srgb=srgb)
+        ctx.save_for_backward(*ins)
+        ctx.kind, ctx.f0, ctx.spec_scale, ctx.srgb = kind, f0, spec_scale, srgb
+        return rgb.reshape(-1, 3)
+
+    @staticmethod
+    def backward(ctx, d_rgb):
+        lvis, normal, albedo, prop, light_flat, xyz, cam, lxyz, lareas = ctx.saved_tensors
+        names = ('lvis', 'normal', 'albedo', 'rough' if ctx.kind == 0 else 'spec', 'light')
+        need = [k for k, want in zip(names, ctx.needs_input_grad[:5]) if want]
+        rough, spec = (prop, None) if ctx.kind == 0 else (None, prop)
+        g = _lib.integrate_bwd(_lib.default_context(), xyz, normal, cam, albedo, lvis, lxyz, lareas,
+                               light_flat, d_rgb.contiguous(), rough=rough, spec=spec, f0=ctx.f0,
+                               spec_scale=ctx.spec_scale, linear2srgb=ctx.srgb, need=need)
+        return tuple(g.get(k) for k in names) + (None,) * 8
+
+
+def integrate(lvis, normal, albedo, brdf_prop, light_flat, xyz, cam, lxyz, lareas, kind, f0,
+              spec_scale, srgb):
+    """Differentiable rendering equation for one env-map (nerfactor.py:212, 315-342 with the BRDF
+    of microfacet.py:30-111 or nerfactor.py:457-461) -> rgb [n, 3].
+    lvis [n, L]; normal [n, 3] raw (normalised here, nerfactor.py:212); albedo [n, 3];
+    brdf_prop: rough [n, 1] (kind 0, microfacet) or the front-masked learned spec [n, L] (kind 1);
+    light_flat [L, 3] (one texel per light, >= 0); xyz / cam [n, 3]; lxyz [L, 3]; lareas [L].
+    CUDA tensors run nf_integrate_fwd / nf_integrate_bwd, which give no gradient for xyz, cam,
+    lxyz or lareas; CPU tensors run the torch composition below."""
+    if lvis.is_cuda:
+        return IntegrateFn.apply(lvis, normal, albedo, brdf_prop, light_flat, xyz, cam, lxyz,
+                                 lareas, kind, f0, spec_scale, srgb)
+    surf2l = safe_l2_normalize(lxyz.reshape(1, -1, 3) - xyz[:, None, :], 2)   # shape.py:128-135
+    surf2c = safe_l2_normalize(cam - xyz, 1)                                  # shape.py:137-144
+    normal = safe_l2_normalize(normal, 1)
+    if kind == 0:
+        brdf = microfacet_brdf(surf2l, surf2c, normal, albedo, brdf_prop, f0)
+    else:
+        n, L = brdf_prop.shape
+        brdf = albedo[:, None, :] / math.pi + (brdf_prop.reshape(n, L, 1) * spec_scale).expand(n, L, 3)
+    return render(lvis, brdf, surf2l, normal, light_flat, lareas, srgb)

@@ -10,7 +10,6 @@ gets its own rays, the per-ray loss is divided by the GLOBAL batch size
 (tf.nn.compute_average_loss, :282-283) and the flat gradient buffer is summed with ONE
 NCCL all-reduce before the optimizer step.
 """
-import math
 
 import numpy as np
 import torch
@@ -160,8 +159,9 @@ class Trainer:
         e = torch.cat((e_x[:, None, :].expand(n, L, e_x.shape[1]).reshape(n * L, -1), e_l), -1)
         return ad.mlp_apply(e, layers, acts, skip, self.precision).reshape(n, L)
 
-    def _brdf_learned(self, surf2l, surf2c, normal, albedo, z):
-        """nerfactor.py:413-461 (all pairs evaluated; back-lit ones are zeroed, :454-455)."""
+    def _brdf_learned(self, surf2l, surf2c, normal, z):
+        """nerfactor.py:413-457 -> the front-masked spec [n, L] (all pairs evaluated; back-lit ones
+        are zeroed, :454-455); albedo / pi + spec * scale (:458-461) is formed by ad.integrate."""
         m = self.model
         n, L = surf2l.shape[0], surf2l.shape[1]
         w2l = ad.gen_world2local(normal)
@@ -176,8 +176,7 @@ class Trainer:
         trunk = m.brdf_model.net['brdf_mlp']
         acts = [l.activation for l in trunk.layers] + ['softplus']
         spec = ad.mlp_apply(e, self.brdf_layers, acts, trunk.skip_at, self.precision)[:, 0] * front
-        scale = m.config.getfloat('DEFAULT', 'learned_brdf_scale')
-        return albedo[:, None, :] / math.pi + (spec.reshape(n, L, 1) * scale).expand(n, L, 3)
+        return spec.reshape(n, L)
 
     def forward(self, flat, batch, mode, xyz_noise=None, all_fg=False):
         """Differentiable `Model.call` (shape.py:146-182 / nerfactor.py:181-313) + loss.
@@ -239,6 +238,7 @@ class Trainer:
             normal_j = None if xyz_j is None else self._point(views, 'normal', xyz_j) + 1e-6
             lvis_pred = self._lvis(views, xyz_m, surf2l)
             lvis_j = None if xyz_j is None else self._lvis(views, xyz_j, surf2l, xyz_m)
+        normal_raw = normal_pred                       # ad.integrate normalises it itself (:212)
         normal_pred = ad.safe_l2_normalize(normal_pred, 1)
         if normal_j is not None:
             normal_j = ad.safe_l2_normalize(normal_j, 1)
@@ -251,17 +251,20 @@ class Trainer:
         if m.normalize_brdf_z:
             z = ad.safe_l2_normalize(z, 1)
             z_j = None if z_j is None else ad.safe_l2_normalize(z_j, 1)
-        if getattr(m, 'brdf_model', None) is not None:
-            brdf = self._brdf_learned(surf2l, surf2c, normal_pred, albedo, z)
-        else:
-            brdf = ad.microfacet_brdf(surf2l, surf2c, normal_pred, albedo, z,
-                                      m.config.getfloat('DEFAULT', 'fresnel_f0'))
         light = torch.clamp(views[('light', 0, 'light')], min=0.)
         light_flat = light.reshape(-1, 3)
         if m.light_idx is not None:
             light_flat = light_flat[m.light_idx.long()]
-        rgb_pred = ad.render(lvis_pred, brdf, surf2l, normal_pred, light_flat, m.lareas,
-                             m.config.getboolean('DEFAULT', 'linear2srgb'))
+        srgb = m.config.getboolean('DEFAULT', 'linear2srgb')
+        if getattr(m, 'brdf_model', None) is not None:
+            spec = self._brdf_learned(surf2l, surf2c, normal_pred, z)
+            rgb_pred = ad.integrate(lvis_pred, normal_raw, albedo, spec, light_flat, xyz_m, rayo_m,
+                                    m.lxyz, m.lareas, 1, 0., m.config.getfloat(
+                                        'DEFAULT', 'learned_brdf_scale'), srgb)
+        else:
+            rgb_pred = ad.integrate(lvis_pred, normal_raw, albedo, z, light_flat, xyz_m, rayo_m,
+                                    m.lxyz, m.lareas, 0, m.config.getfloat('DEFAULT', 'fresnel_f0'),
+                                    1., srgb)
         pred = {'rgb': scatter(rgb_pred), 'normal': scatter(normal_pred),
                 'lvis': scatter(lvis_pred), 'albedo': scatter(albedo), 'brdf': scatter(z)}
         gt = {'rgb': scatter(rgb_m), 'normal': scatter(normal_m), 'lvis': scatter(lvis_m),
